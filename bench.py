@@ -3,6 +3,8 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]                 our CUDA path (liburf_b200.so through the C-ABI)
   python bench.py --impl reference [--gpus N] [--steps K] [--warmup W] the reference's own CPU implementation, host cores
+  python bench.py ... --dump-outputs DIR                               also writes what the last timed step computed
+                                                                       (dump_outputs), to compare two builds
 
 A "step" is one pass of the hot path over one batch of `--batch` distinct synthetic OS1-64 scans (BASELINE config 2:
 64 rings x 2048 columns = 131,072 points per scan, all three detectors + blindSpots, full-ROI preset so every point
@@ -225,6 +227,33 @@ def ncu_traffic(kernel: str):
     return None
 
 
+DUMP_MAX_LABELS = 1 << 23          # 32 MiB of float32 labels per process; larger outputs are sampled
+COUNT_FIELDS = ("status", "n_in", "n_roi", "n_rings", "n_order", "n_road", "n_curb", "n_vert", "flags")
+
+
+def dump_outputs(path: str, labels, outs, rank: int, world: int) -> None:
+    """Writes what one device-resident step returned to its caller, so two builds can be compared output for output:
+    label.npy  float32 labels of the (batch, points) label array, flattened; all of them when there are at most
+               DUMP_MAX_LABELS / world, else that many at flat positions drawn with seed 0 (the same for the same arguments);
+    counts.npy float64 (batch, 9): the per-scan counts of urf_result (COUNT_FIELDS);
+    vert.npy   float32 (batch, URF_MAX_VERTS, 4): the marker candidate vertices, rows past n_vert zeroed.
+    With several ranks each writes its own files, suffixed _rank<r>."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    sfx = f"_rank{rank}" if world > 1 else ""
+    flat = labels.reshape(-1)
+    cap = DUMP_MAX_LABELS // world
+    if flat.numel() > cap:
+        idx = np.sort(np.random.default_rng(0).choice(flat.numel(), size=cap, replace=False))
+        flat = flat[torch.from_numpy(idx).to(flat.device)]
+    np.save(os.path.join(path, f"label{sfx}.npy"), flat.cpu().numpy().astype(np.float32))
+    np.save(os.path.join(path, f"counts{sfx}.npy"), np.array([[getattr(o, f) for f in COUNT_FIELDS] for o in outs], np.float64))
+    vert = np.stack([np.ctypeslib.as_array(o.vert).copy() for o in outs]).astype(np.float32)
+    for b, o in enumerate(outs):
+        vert[b, o.n_vert:] = 0.0
+    np.save(os.path.join(path, f"vert{sfx}.npy"), vert)
+
+
 # ----------------------------------------------------------------------------------------------------------------------
 def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
@@ -282,10 +311,17 @@ def main():
     ap.add_argument("--no-xzero", action="store_true", help="detector ablation: x_zero_method off")
     ap.add_argument("--no-zzero", action="store_true", help="detector ablation: z_zero_method off")
     ap.add_argument("--no-with-order", action="store_true", help="skip the second timed pass that also produces the emission order")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the labels (sampled above 2^23), per-scan counts and vertices of the "
+                         "last device-resident step as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "urf" else args.warmup
     if args.steps is None:
         args.steps = 200 if args.impl == "urf" else 10
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "urf" or args.sweep):
+        ap.error("--dump-outputs writes the outputs of the timed device-resident path: not with --impl reference or --sweep")
     for flag, key in ((args.no_star, "star_shaped_method"), (args.no_xzero, "x_zero_method"), (args.no_zzero, "z_zero_method")):
         if flag:
             _ABLATION[key] = 0
@@ -402,6 +438,8 @@ def main():
     t_w1 = time.time()
     dev_ms = e0.elapsed_time(e1)
     assert lib.urf_finish_batch_device(ctx, outs) == 0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, labels, outs, rank, world)
     launches = det.last_launch_count() * args.steps
     n_road = sum(o.n_road for o in outs)
     # ---- timed region 1w: the same K steps with the per-ring azimuth sort (lidar_segmentation.cpp:289-291) and the emission

@@ -1,13 +1,17 @@
-"""Generates tests/golden/*.npz by running the UNMODIFIED reference (oracle/_ref/liburf_ref.so, built from
-/root/reference/src by `make -C oracle ref`) on seeded synthetic clouds. Run here, in the build container; the fixtures
-travel to the GPU box where /root/reference does not exist.
+"""Generates tests/golden/*.npz by running the UNMODIFIED reference (oracle/_ref/liburf_ref.so, built from the
+reference's sources by `make -C oracle ref REF=<reference checkout>`) on seeded synthetic clouds. Needs the reference
+build; the fixtures let the tests compare with the reference wherever it cannot be built.
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py [--only <name prefix>]
 
 Each fixture holds: params (cfg overrides), the input cloud (or, for big clouds, the generator recipe + sha256 of the
 bytes it must produce), and what the reference published: per-point labels (recovered from the roi/road/curb clouds),
 the road / curb / road_probably clouds as input-index lists in emission order, and the road_marker line strips with
 simplification off (exact vertices) and with the cfg defaults.
+
+tests/golden/ref_runs/<family>.npz (name prefix "ref_runs") hold the reference's results on the cases of the tests that
+compare with it directly (util.StoredRefRuns): the seeded random parameter draws of tests/test_oracle.py, the marker
+strips of tests/test_markers.py and the labels of scripts/fuzz_model.py's first 60 seeds.
 """
 from __future__ import annotations
 
@@ -21,10 +25,14 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+sys.path.insert(0, os.path.join(ROOT, "scripts"))
 
-from oracle.pyoracle import RefOracle  # noqa: E402
+from fuzz_model import fuzz_case, fuzz_key, ref_compares, run_ref_isolated  # noqa: E402
+from oracle.pyoracle import RefOracle, RefResult  # noqa: E402
 from urban_road_filter_b200 import FULL_ROI, make_params  # noqa: E402
 from urban_road_filter_b200.synth import SHAPES, make_scan, random_cloud  # noqa: E402
+from util import MARKER_EPS, REF_RUNS_DIR, marker_case, random_params_case, ref_run_digest  # noqa: E402
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 
@@ -69,9 +77,52 @@ def strips_to_arrays(strips):
     return meta, pts.astype(np.float64)
 
 
+def ref_run_arrays(key: str, pts, prm, r, fields) -> dict:
+    """One case of a ref_runs family: the digest of its inputs, whether the reference crashed, and `fields` of its result."""
+    out = {f"{key}.digest": np.array(ref_run_digest(pts, prm)), f"{key}.crashed": np.int8(r is None)}
+    for f in fields if r is not None else ():
+        if f == "strips":
+            out[f"{key}.strips_meta"], out[f"{key}.strips_pts"] = strips_to_arrays(r.strips)
+        elif f == "label":
+            out[f"{key}.label"] = r.label.astype(np.int8)
+        else:
+            out[f"{key}.{f}"] = np.asarray(getattr(r, f))
+    return out
+
+
+def make_ref_runs(ref: RefOracle):
+    os.makedirs(REF_RUNS_DIR, exist_ok=True)
+    runs = {}
+    for seed in range(6):
+        pts, prm = random_params_case(seed)
+        runs.update(ref_run_arrays(str(seed), pts, prm, ref.run(pts, prm), ("published", "label", "road_ids", "curb_ids")))
+    np.savez_compressed(os.path.join(REF_RUNS_DIR, "random_params.npz"), **runs)
+    runs = {}
+    for seed in range(4):
+        for k, eps in enumerate(MARKER_EPS):
+            pts, prm = marker_case(seed, eps)
+            runs.update(ref_run_arrays(f"{seed}_{k}", pts, prm, ref.run(pts, prm, ghostcount=0), ("markers_published", "strips")))
+    np.savez_compressed(os.path.join(REF_RUNS_DIR, "markers.npz"), **runs)
+    runs = {}
+    for seed in range(60):
+        _, pts, prm = fuzz_case(seed)
+        if ref_compares(pts.shape[0], False):
+            label = run_ref_isolated(ref, pts, prm)
+            r = None
+            if label is not None:
+                r = RefResult()
+                r.label = label
+            runs.update(ref_run_arrays(fuzz_key(seed), pts, prm, r, ("label",)))
+    np.savez_compressed(os.path.join(REF_RUNS_DIR, "fuzz.npz"), **runs)
+    print(f"ref_runs: {len(runs)} arrays of fuzz cases, sizes " +
+          ", ".join(f"{f} {os.path.getsize(os.path.join(REF_RUNS_DIR, f))} B" for f in sorted(os.listdir(REF_RUNS_DIR))))
+
+
 def main():
     only = sys.argv[sys.argv.index("--only") + 1] if "--only" in sys.argv else ""      # name prefix; default: everything but c5
     ref = RefOracle()
+    if "ref_runs".startswith(only):
+        make_ref_runs(ref)
     env = dict(machine=platform.machine(), libc=" ".join(platform.libc_ver()), python=platform.python_version(),
                numpy=np.__version__)
     for name, recipe, store, over in CASES:

@@ -5,8 +5,10 @@ reference tree, so `simplify` is PARITY UNPINNED (DESIGN.md): the product states
 import numpy as np
 import pytest
 
-from oracle.pyoracle import RefOracle
+from oracle.pyoracle import PortOracle
 from urban_road_filter_b200 import api, make_params
+
+from util import MARKER_EPS, StoredRefRuns, marker_case
 
 
 def strip_points(vert_xy, eps, simplify=True):
@@ -77,21 +79,17 @@ def test_simplify_collinear_and_degenerate():
     assert len(strip_points(closed, 0.7)) == 3
 
 
-@pytest.mark.skipif(not RefOracle.available(), reason="oracle/_ref is built from /root/reference (this container only)")
 @pytest.mark.parametrize("seed", range(4))
 def test_iterative_and_recursive_statements_agree(seed):
     """The product (iterative) against the reference build, whose marker tail (the unmodified lidar_segmentation.cpp:369-602)
-    calls the shim's recursive statement: same strips for the same candidate vertices, at several tolerances."""
-    from urban_road_filter_b200 import FULL_ROI
-    from urban_road_filter_b200.synth import make_scan
-    ref = RefOracle()
-    pts = make_scan("C1", 20 + seed)
-    for eps in (0.05, 0.7, 3.0):
-        prm = make_params(poly_s_param=eps, **FULL_ROI)
-        r = ref.run(pts, prm, ghostcount=0)
+    calls the shim's recursive statement: same strips for the same candidate vertices, at several tolerances. The
+    reference's strips are stored in tests/golden/ref_runs/markers.npz."""
+    stored = StoredRefRuns("markers")
+    for k, eps in enumerate(MARKER_EPS):
+        pts, prm = marker_case(seed, eps)
+        r = stored.run(f"{seed}_{k}", pts, prm)
         if not r.markers_published:
             continue
-        from oracle.pyoracle import PortOracle
         o = PortOracle().run(pts, prm)
         mine, _ = api.build_markers(prm, o.vert, 0)
         assert len(mine) == len(r.strips)

@@ -12,7 +12,7 @@ from urban_road_filter_b200 import FULL_ROI, make_params
 from urban_road_filter_b200.api import build_markers
 from urban_road_filter_b200.synth import SHAPES, make_scan, random_cloud
 
-from util import CpuModel, Golden, assert_matches_golden, golden_names, stage_diffs
+from util import CpuModel, Golden, StoredRefRuns, assert_matches_golden, golden_names, stage_diffs
 
 
 @pytest.fixture(scope="module")
@@ -82,12 +82,15 @@ def test_model_zero_elevation_quirk(both):
 
 
 def test_model_fuzz_short():
-    """A short run of scripts/fuzz_model.py (random parameter draws x varied clouds; model vs port and vs the unmodified
-    reference where it is built). The long run (3000 cases, 0 mismatches) is recorded in DESIGN.md §2."""
+    """A short run of scripts/fuzz_model.py (random parameter draws x varied clouds; model vs port, and vs the unmodified
+    reference's labels stored for these seeds). The long run (3000 cases, 0 mismatches) is recorded in DESIGN.md §2."""
     import os
+    import re
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     out = subprocess.run([sys.executable, os.path.join(root, "scripts", "fuzz_model.py"), "0", "60"], capture_output=True, text=True, timeout=900)
     assert out.returncode == 0, out.stderr[-2000:]
     assert "mismatching cases 0;" in out.stdout, out.stdout[-2000:]
+    m = re.search(r"(\d+) of them also vs the unmodified reference, (\d+) reference crashes", out.stdout)
+    assert m and int(m.group(1)) > 0 and int(m.group(1)) + int(m.group(2)) == len(StoredRefRuns("fuzz")), out.stdout[-2000:]

@@ -1,14 +1,15 @@
 """The oracle itself: the CPU restatement (oracle/urf_oracle.cpp) is pinned against the golden fixtures generated from the
-UNMODIFIED reference (tests/golden/make_golden.py) and, where oracle/_ref exists, against the reference directly."""
+UNMODIFIED reference (tests/golden/make_golden.py) and against the reference's stored results on seeded random parameter
+draws (tests/golden/ref_runs/random_params.npz)."""
 import numpy as np
 import pytest
 
-from oracle.pyoracle import PortOracle, RefOracle
+from oracle.pyoracle import PortOracle
 from urban_road_filter_b200 import FULL_ROI, make_params
 from urban_road_filter_b200.api import build_markers
-from urban_road_filter_b200.synth import make_scan, random_cloud
+from urban_road_filter_b200.synth import make_scan
 
-from util import Golden, assert_matches_golden, golden_names
+from util import Golden, StoredRefRuns, assert_matches_golden, golden_names, random_params_case
 
 
 @pytest.fixture(scope="module")
@@ -23,22 +24,11 @@ def test_port_matches_reference_golden(port, name):
     assert_matches_golden(g, r, build_markers)
 
 
-@pytest.mark.skipif(not RefOracle.available(), reason="oracle/_ref not built (no /root/reference on this box)")
 @pytest.mark.parametrize("seed", range(6))
 def test_port_matches_reference_random_params(port, seed):
     """Seeded random draws over the LidarFilters.cfg parameter ranges (cfg/LidarFilters.cfg:10-84)."""
-    ref = RefOracle()
-    rng = np.random.default_rng(100 + seed)
-    pts = make_scan("C1", 10 + seed, order=("column", "ring")[seed % 2]) if seed % 3 else random_cloud(6000, seed, rings=12)
-    prm = make_params(
-        x_zero_method=int(rng.integers(0, 2)), z_zero_method=int(rng.integers(0, 2)), star_shaped_method=int(rng.integers(0, 2)),
-        blind_spots=int(rng.integers(0, 2)), xDirection=int(rng.integers(0, 3)), interval=float(rng.uniform(0.05, 0.5)),
-        curb_height=float(rng.uniform(0.01, 0.2)), curb_points=int(rng.integers(1, 12)), beamZone=float(rng.uniform(10, 100)),
-        cylinder_deg_x=float(rng.uniform(90, 180)), cylinder_deg_z=float(rng.uniform(90, 180)),
-        curb_slope_deg=float(rng.uniform(10, 90)), kdev_param=float(rng.uniform(0.5, 5)), kdist_param=float(rng.uniform(0.4, 10)),
-        starbeam_filter=int(rng.integers(0, 2)), dmin_param=int(rng.integers(3, 30)),
-        **(FULL_ROI if seed % 2 else dict(min_x=-20.0, max_x=40.0, min_y=-15.0, max_y=15.0, min_z=-3.0, max_z=1.0)))
-    r = ref.run(pts, prm)
+    pts, prm = random_params_case(seed)
+    r = StoredRefRuns("random_params").run(str(seed), pts, prm)
     p = port.run(pts, prm)
     assert r.published == (p.status == 0)
     if r.published:

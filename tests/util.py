@@ -14,12 +14,13 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-from oracle.pyoracle import OracleDebug  # noqa: E402
-from urban_road_filter_b200 import UrfParams, UrfResult, make_params  # noqa: E402
+from oracle.pyoracle import OracleDebug, RefResult  # noqa: E402
+from urban_road_filter_b200 import FULL_ROI, UrfParams, UrfResult, make_params  # noqa: E402
 from urban_road_filter_b200.ctypes_abi import URF_MAX_CHANNELS, URF_MAX_VERTS  # noqa: E402
 from urban_road_filter_b200.synth import make_scan, random_cloud  # noqa: E402
 
 GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
+REF_RUNS_DIR = os.path.join(GOLDEN_DIR, "ref_runs")
 VERT_TOL = 1e-4     # metres: BASELINE.json north_star tolerance for curb-polyline vertices
 
 
@@ -109,6 +110,73 @@ def compare_strips(mine, ref, what):
         assert a[2] == b[2], f"{what}: colour"
         assert a[3].shape == b[3].shape, f"{what}: strip {a[0]} has {a[3].shape[0]} points, reference {b[3].shape[0]}"
         assert np.all(np.abs(a[3] - b[3]) <= VERT_TOL), f"{what}: vertex off by {np.abs(a[3] - b[3]).max()} m"
+
+
+def random_params_case(seed: int):
+    """(cloud, parameters) of seeded random draw `seed` over the LidarFilters.cfg parameter ranges (cfg/LidarFilters.cfg:10-84)."""
+    rng = np.random.default_rng(100 + seed)
+    pts = make_scan("C1", 10 + seed, order=("column", "ring")[seed % 2]) if seed % 3 else random_cloud(6000, seed, rings=12)
+    prm = make_params(
+        x_zero_method=int(rng.integers(0, 2)), z_zero_method=int(rng.integers(0, 2)), star_shaped_method=int(rng.integers(0, 2)),
+        blind_spots=int(rng.integers(0, 2)), xDirection=int(rng.integers(0, 3)), interval=float(rng.uniform(0.05, 0.5)),
+        curb_height=float(rng.uniform(0.01, 0.2)), curb_points=int(rng.integers(1, 12)), beamZone=float(rng.uniform(10, 100)),
+        cylinder_deg_x=float(rng.uniform(90, 180)), cylinder_deg_z=float(rng.uniform(90, 180)),
+        curb_slope_deg=float(rng.uniform(10, 90)), kdev_param=float(rng.uniform(0.5, 5)), kdist_param=float(rng.uniform(0.4, 10)),
+        starbeam_filter=int(rng.integers(0, 2)), dmin_param=int(rng.integers(3, 30)),
+        **(FULL_ROI if seed % 2 else dict(min_x=-20.0, max_x=40.0, min_y=-15.0, max_y=15.0, min_z=-3.0, max_z=1.0)))
+    return pts, prm
+
+
+MARKER_EPS = (0.05, 0.7, 3.0)
+
+
+def marker_case(seed: int, eps: float):
+    """(cloud, parameters) of a whole VLP-16 scan whose road_marker strips are simplified with tolerance `eps`."""
+    return make_scan("C1", 20 + seed), make_params(poly_s_param=eps, **FULL_ROI)
+
+
+def ref_run_digest(pts: np.ndarray, prm: UrfParams) -> str:
+    """sha256 of a cloud's bytes and of every parameter value: names the inputs a stored reference run was made on."""
+    h = hashlib.sha256(np.ascontiguousarray(pts, np.float32).tobytes())
+    h.update(repr([getattr(prm, f) for f, _ in UrfParams._fields_]).encode())
+    return h.hexdigest()
+
+
+class StoredRefRuns:
+    """What the unmodified reference (oracle.pyoracle.RefOracle.run) returned on named cases, recorded by
+    tests/golden/make_golden.py into tests/golden/ref_runs/<family>.npz, so that comparisons with the reference also run
+    where it cannot be built. Each case holds the digest of its inputs and the fields its tests compare."""
+
+    def __init__(self, family: str):
+        z = np.load(os.path.join(REF_RUNS_DIR, family + ".npz"))
+        self._cases: dict[str, dict] = {}
+        for f in z.files:
+            key, field = f.rsplit(".", 1)
+            self._cases.setdefault(key, {})[field] = z[f]
+
+    def __contains__(self, key: str) -> bool:
+        return key in self._cases
+
+    def __len__(self) -> int:
+        return len(self._cases)
+
+    def run(self, key: str, pts: np.ndarray, prm: UrfParams):
+        """The stored RefOracle().run(pts, prm) of case `key`, or None where the reference crashed on it."""
+        a = self._cases[key]
+        assert str(a["digest"]) == ref_run_digest(pts, prm), f"{key}: not the cloud and parameters the reference was run on"
+        if a["crashed"]:
+            return None
+        r = RefResult()
+        for f, v in a.items():
+            if f in ("published", "markers_published"):
+                setattr(r, f, bool(v))
+            elif f == "label":
+                r.label = v.astype(np.int32)
+            elif f not in ("digest", "crashed", "strips_meta", "strips_pts"):
+                setattr(r, f, v)
+        if "strips_meta" in a:
+            r.strips = Golden._strips(a["strips_meta"], a["strips_pts"])
+        return r
 
 
 def feq(a: np.ndarray, b: np.ndarray) -> bool:

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Registers / spills / shared memory per kernel (ptxas -v) and the Blackwell/Hopper-class SASS mnemonics each kernel
-contains (cluster barriers UCGABAR_*, distributed-shared-memory mapping, warp REDUX, MATCH, 64-bit shared atomics).
+contains (warp REDUX, MATCH, 64-bit shared atomics; cluster barriers UCGABAR_* would show up here).
 usage: python scripts/ptxas_table.py > profiles/r02_ptxas_sass_<version>.txt   (no GPU needed: nvcc cross-compiles)"""
 import os, re, subprocess, sys, collections
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -34,6 +34,5 @@ for name, regs, stack, sst, sld, smem in sorted(rows):
     c = per.get(name, {})
     notes = ", ".join(f"{k} {v}" for k, v in sorted(c.items()) if k != "total" and k not in ("DFMA", "DMUL", "DADD") and v)
     print(f"{name:28s} {regs:4d} {stack:5d} {sst:8d} {sld:8d} {smem:7d} {c.get('total', 0):6d}  {notes}")
-print("\nUCGABAR_ARV / UCGABAR_WAIT = thread-block-cluster barrier (cluster.sync); ATOM on generic addresses in k_markers target the")
-print("shared memory of the cluster's first CTA (distributed shared memory, cluster.map_shared_rank); REDUX = warp-wide integer reduce;")
-print("MATCH = __match_any_sync. No tensor-core or TMA instructions: the path has no dense contraction and no bulk tile to stage.")
+print("\nREDUX = warp-wide integer reduce; MATCH = __match_any_sync. No tensor-core or TMA instructions: the path has no dense")
+print("contraction and no bulk tile to stage.")

@@ -1,21 +1,18 @@
-"""Small scans through the code paths added in round 2, for compute-sanitizer: the marker search variants (cluster with
-distributed shared memory / one CTA / grid), both ring detectors, the emission-order counting sort and its fallback, the
-radius-tie path (restated std::sort by one thread), the registration repair inside k_scan_offsets, the lean and record entries."""
+"""Small scans through the code paths added in round 2, for compute-sanitizer: both marker searches (one CTA per scan /
+a grid of CTAs for scans above 300 k points), both ring detectors, the emission-order counting sort and its fallback,
+the radius-tie path (restated std::sort by one thread), the registration repair inside k_scan_offsets, the lean and record
+entries."""
 import sys
 sys.path.insert(0, ".")
 import numpy as np
+from oracle.pyoracle import PortOracle
 from urban_road_filter_b200 import api, make_params, FULL_ROI
-from urban_road_filter_b200.synth import make_scan, random_cloud
+from urban_road_filter_b200.synth import SHAPES, make_scan, random_cloud
 
 prm = make_params(**FULL_ROI)
 pts = make_scan("C1", 3)
 det = api.Detector(max_points=30000, max_batch=4, params=prm)
 base = det.filtered(pts)
-for rd, mk in ((46, 1), (4, 0), (8, 2), (45, 0)):
-    det.set_option(8, rd); det.set_option(9, mk)
-    r = det.filtered(pts)
-    assert np.array_equal(r.label, base.label) and np.array_equal(r.order, base.order) and np.array_equal(r.vert, base.vert), (rd, mk)
-det.set_option(8, 46); det.set_option(9, 1)
 tie = pts.copy(); tie[1000:1300, :3] = tie[3000:3300, :3]                      # equal radii -> std::sort emulation
 assert det.filtered(tie).flags & 2
 assert det.filtered(random_cloud(5000, 5)).flags & 1                            # speculation refuted -> repair in k_scan_offsets
@@ -25,9 +22,6 @@ rs = det.filtered_batch_records([np.ascontiguousarray(pts[:, :3]), np.ascontiguo
 assert np.array_equal(rs[0].label, base.label)
 flat = make_scan("C1", 4).copy(); flat[:, 2] = -1.8                              # no edges: every sector refined
 det.filtered(flat)
-det.set_option(12, 32); r32 = det.filtered(pts); det.set_option(12, 16)          # single-warp star sort at 32 elements per lane
-det.set_option(11, 0); r1s = det.filtered(pts); det.set_option(11, 1)            # ring detector on the pipeline's own stream
-assert np.array_equal(r32.label, base.label) and np.array_equal(r1s.label, base.label)
 det.close()
 # OS1-64 sectors (364 points) are sorted near-first; in a flat / half-flat world the walks run off the prefix:
 # k_star_refine (remainder sort behind the prefix + warp-wide resumed walk) on every / every other sector
@@ -40,5 +34,15 @@ for variant in ("flat", "half"):
     a = det.filtered(w)
     det.set_option(4, 0); b = det.filtered(w); det.set_option(4, 1)             # whole-sector sorting: same result
     assert np.array_equal(a.label, b.label) and np.array_equal(a.order, b.order), variant
+det.close()
+# a scan above 300 k points: the grid marker search (k_markers_grid x 2 + k_verts), against the CPU oracle
+sh = SHAPES["C5"]
+cut = make_scan("C5", 6)[:320000]
+prm5 = make_params(channels=sh.channels, interval=sh.interval, **FULL_ROI)
+det = api.Detector(max_points=cut.shape[0], max_batch=1, params=prm5)
+r = det.filtered(cut)
+o = PortOracle().run(cut, prm5)
+assert r.status == o.status == 0 and np.array_equal(r.label, o.label)
+assert r.n_vert == o.n_vert and np.array_equal(r.vert, o.vert)
 print("ok")
 det.close()

@@ -277,7 +277,7 @@ extern "C" int urf_model_run(const float* xyzi, int n, const urf_params* up, urf
   }
 
   // ---- k_label (input order), k_dmax, k_best, k_verts
-  std::vector<unsigned> dmax(kDegBins, 0u);                     // k_markers keeps these two in the cluster's shared memory
+  std::vector<unsigned> dmax(kDegBins, 0u);                     // k_markers1 keeps these two in its shared memory
   std::vector<unsigned long long> best(kDegBins, ~0ull);
   for (int i = 0; i < kDegBins; i++) tab.cutbest[i] = ~0ull;
   int formulation_mismatch = 0;

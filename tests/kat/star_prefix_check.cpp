@@ -58,7 +58,7 @@ int main(int argc, char** argv) {
     for (int l = 0; l < 32; l++) {
       int rank = 0;
       for (int j = 0; j < 32; j++) rank += (samples[j] < samples[l]) || (samples[j] == samples[l] && j < l);
-      if (rank == 17) pivot = samples[l];
+      if (rank == kStarPivot) pivot = samples[l];
     }
     std::vector<float4> near;
     for (const float4& p : pts) if (fbits(p.x) < pivot) near.push_back(p);

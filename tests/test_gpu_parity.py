@@ -10,6 +10,7 @@ import torch
 from oracle.pyoracle import PortOracle
 from urban_road_filter_b200 import FULL_ROI, make_params
 from urban_road_filter_b200 import api
+from urban_road_filter_b200.ctypes_abi import URF_ERR_INVALID
 from urban_road_filter_b200.synth import SHAPES, make_scan, random_cloud
 
 from util import Golden, assert_matches_golden, golden_names, stage_diffs
@@ -522,15 +523,14 @@ def test_gpu_packed_clouds_match_oracle(det, port, shape, step, offs):
         assert r.label is None and (r.n_road, r.n_curb) == (len(exp["road"]), len(exp["curb"]))
 
 
-SORT_WIDTH_DEFAULT = 16
-
-
 @pytest.mark.parametrize("variant", ["scan", "flat", "half_flat"])
-@pytest.mark.parametrize("shape", ["C2", "C4"])
+@pytest.mark.parametrize("shape", ["C1", "C2", "C3", "C4"])
 def test_gpu_near_first_star_sort(det, port, shape, variant):
     """k_star_sort_warp sorts only the points below a sampled pivot radius and k_star_scan redoes (tab.refine) the sectors
     whose edge search runs off that prefix. A flat world has no edge at all (every sector is refined), a half-flat one
-    mixes both paths; each must give the oracle's result, and the same result as whole-sector sorting (option 4 = 0)."""
+    mixes both paths; each must give the oracle's result, and the same result as whole-sector sorting (option 4 = 0).
+    Typical star sectors: about 80 points (C1: below the near-first threshold), 380 (C2, C3) and 760 (C4: whole-sector
+    sorts of more than 512 points go to k_star_sort_big)."""
     sh = SHAPES[shape]
     pts = make_scan(shape, 31)
     if variant == "flat":
@@ -544,14 +544,27 @@ def test_gpu_near_first_star_sort(det, port, shape, variant):
     if variant == "flat":
         assert int((np.asarray(o.star_mark) == 2).sum()) == 0
     res = {}
-    for mode, width in ((1, 16), (0, 16), (1, 32), (0, 32)):   # option 12: widest single-warp network (wider sorts: k_star_sort_big)
+    for mode in (1, 0):
         det.set_option(4, mode)
-        det.set_option(12, width)
         r = det.filtered(pts)
-        assert stage_diffs(o, GpuDebug(det, r, n), n) == [], f"star_prefix={mode} width={width}"
-        res[mode, width] = r
+        assert stage_diffs(o, GpuDebug(det, r, n), n) == [], f"star_prefix={mode}"
+        res[mode] = r
     det.set_option(4, 1)
-    det.set_option(12, SORT_WIDTH_DEFAULT)
-    for k in res:
-        np.testing.assert_array_equal(res[k].label, res[1, 32].label)
-        np.testing.assert_array_equal(res[k].vert, res[1, 32].vert)
+    np.testing.assert_array_equal(res[0].label, res[1].label)
+    np.testing.assert_array_equal(res[0].vert, res[1].vert)
+
+
+# options 5-12 selected tuning variants that were removed: each accepts only the value now built in
+RETIRED_OPTIONS = {5: 0, 6: 0, 7: 0, 8: 46, 9: 1, 10: 17, 11: 1, 12: 16}
+
+
+def test_gpu_retired_options(det):
+    """A retired option set to its built-in value is accepted, so old tuning command lines keep working; asking for a
+    removed variant is refused with URF_ERR_INVALID instead of silently running the built-in one."""
+    for opt, builtin in RETIRED_OPTIONS.items():
+        det.set_option(opt, builtin)
+    removed = ((5, 4), (6, 1), (7, 1), (8, 4), (8, 8), (9, 0), (9, 2), (10, 14), (11, 0), (12, 32))
+    for opt, value in removed:
+        with pytest.raises(api.UrfError) as e:
+            det.set_option(opt, value)
+        assert e.value.code == URF_ERR_INVALID, (opt, value)

@@ -3,7 +3,6 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <string>
 #include <vector>
@@ -25,23 +24,11 @@ struct urf_ctx {
   cudaStream_t s_grp[kGroups] = {};               // independent, so their (short, partly latency-bound) kernels overlap
   cudaEvent_t ev_fork = nullptr, ev_join[kGroups] = {};
   // inside one pipeline the star-shaped search (four kernels) and the ring detector (one kernel) are independent between
-  // k_scatter and k_tab1: with `inner_fork` the ring detector runs on a side stream of the pipeline's stream (tuning option 11)
+  // k_scatter and k_tab1: the ring detector runs on a side stream of the pipeline's stream (measured at C2 x 128:
+  // 1.240 -> 1.233 ms on two streams, 1.282 -> 1.263 on one)
   cudaStream_t s_side[kGroups + 1] = {};
   cudaEvent_t ev_sfork[kGroups + 1] = {}, ev_sjoin[kGroups + 1] = {};
-  bool inner_fork = true;              // measured at C2 x 128: 1.240 -> 1.233 ms on two streams, 1.282 -> 1.263 on one
-  int sort_variant = 16;               // widest single-warp network of k_star_sort_warp in elements per lane: 16 (64 registers, 32 warps/SM)
-                                       // or 32 (128 registers, 16 warps/SM; measured 2 % slower per step at C2 x 128) (tuning option 12)
   int groups = 2;                                 // measured at C2 x 128: 1 stream 1.37 ms, 2 streams 1.31, 4 streams 1.34, 8 streams 1.40
-  // device-resident batches as many small sub-batches: `sub` scans per sub-batch (0 = one sub-batch per stream), dealt
-  // round-robin to the `groups` streams, the whole fork/join captured once as a CUDA graph (bgraph) and replayed; with
-  // `slot_reuse` the sub-batches of a stream share one workspace slot (working set = groups * sub scans, L2-resident)
-  int sub = 0;
-  int markers_variant = 1;             // 0: cluster of eight CTAs per scan (k_markers), 1: one CTA per scan (k_markers1) (tuning option 9)
-  int rd_variant = 46;                 // 4 / 45 / 46: k_ring_detect4 (four positions per thread; default curb_points only) at 4 / 5 / 6 CTAs per SM;
-                                       // 8 / 6 / 5: k_ring_detect (one position per thread) (tuning option 8)
-  bool slot_reuse = false, batch_graph = false;
-  cudaGraphExec_t bexec = nullptr;
-  struct { int B = -1, S = -1, sub = -1, G = -1, order = -1; bool reuse = false; const void* in = nullptr; void* label = nullptr; void* orderp = nullptr; unsigned long long version = 0; int launches = 0; } bkey;
   // CUDA graph of the kernel sequence for small host-buffer batches (launch latency dominates there); re-captured when
   // the shape, the parameters or an option change
   bool use_graph = true;
@@ -116,25 +103,23 @@ __global__ void k_ring32(DevBuffers buf, int* dst, int S) {
   if (i < buf.n[b]) dst[(size_t)b * S + i] = max((int)buf.ringid[(size_t)b * S + i], -1);
 }
 
-// View of `buf` for a sub-batch: what belongs to a scan for good (input, labels, point count, results, emission order) is
-// advanced by b0 scans, the workspace arrays by w0 scans (S points of stride, T histogram rows per scan). w0 == b0 gives
-// every scan its own workspace; sub-batches that run one after the other on one stream may share a slot (w0 = slot * sub).
-DevBuffers slot_view(const DevBuffers& a, int b0, int w0, int S, int T, int channels) {
+// View of `buf` for the scans from b0 on: every per-scan array, the workspace included, is advanced by b0 scans (S points
+// of stride, T histogram rows per scan).
+DevBuffers offset_view(const DevBuffers& a, int b0, int S, int T, int channels) {
   DevBuffers v = a;
-  const size_t o = (size_t)b0 * S, w = (size_t)w0 * S;
+  const size_t o = (size_t)b0 * S;
   v.in += o; v.label += o; v.order += o; v.n += b0; v.out += b0;
   if (v.label8) v.label8 += o;
-  v.alpha_v += w; v.mark += w; v.ringid += w; v.sect += w; v.bpt += w; v.spt += w; v.ssorted += w;
-  v.az += w; v.d2 += w; v.baz += w; v.roadlist += w; v.roadcnt += (size_t)w0 * ((S + 31) >> 5); v.sortbuf += 2 * w;
-  v.Tf += (size_t)w0 * channels * kTStride; v.Tb += (size_t)w0 * channels * kTStride;
-  v.lut += (size_t)w0 * (kElevBins + 1); v.firstidx += (size_t)w0 * (kElevBins + 1);
-  v.hist += (size_t)w0 * T * kRingKeys;
-  v.cmin += (size_t)w0 * channels * kDegBins; v.cmax += (size_t)w0 * channels * kDegBins;
-  v.ne += (size_t)w0 * channels * (kDegBins + 1);
-  v.tab += w0;
+  v.alpha_v += o; v.mark += o; v.ringid += o; v.sect += o; v.bpt += o; v.spt += o; v.ssorted += o;
+  v.az += o; v.d2 += o; v.baz += o; v.roadlist += o; v.roadcnt += (size_t)b0 * ((S + 31) >> 5); v.sortbuf += 2 * o;
+  v.Tf += (size_t)b0 * channels * kTStride; v.Tb += (size_t)b0 * channels * kTStride;
+  v.lut += (size_t)b0 * (kElevBins + 1); v.firstidx += (size_t)b0 * (kElevBins + 1);
+  v.hist += (size_t)b0 * T * kRingKeys;
+  v.cmin += (size_t)b0 * channels * kDegBins; v.cmax += (size_t)b0 * channels * kDegBins;
+  v.ne += (size_t)b0 * channels * (kDegBins + 1);
+  v.tab += b0;
   return v;
 }
-DevBuffers offset_view(const DevBuffers& a, int b0, int S, int T, int channels) { return slot_view(a, b0, b0, S, T, channels); }
 
 constexpr int kMaxKernels = 32;
 constexpr int kMarkSingleMax = 300000;   // scans above this many points take the multi-CTA marker search
@@ -170,7 +155,7 @@ int launch_pipeline(urf_ctx* ctx, const DevBuffers& buf, int B, int S, bool want
   K("k_scatter", k_scatter<<<gchunk, kWarpsPerBlock * 32, 0, st>>>(buf, dp, S, T));   // 64 registers, 4 CTAs/SM (48 / 40 registers spill: measured slower)
   // the ring detector next to the star-shaped search: both only read what k_scatter left and add curb hits (idempotent
   // marks, atomic min / max aggregates); k_tab1 is the first reader of the aggregates
-  const bool fork = ctx->inner_fork && dp.star && !ctx->profile;
+  const bool fork = dp.star && !ctx->profile;
   cudaStream_t st_ring = st;
   int side = urf_ctx::kGroups;
   if (fork) {
@@ -183,21 +168,15 @@ int launch_pipeline(urf_ctx* ctx, const DevBuffers& buf, int B, int S, bool want
   {
     cudaStream_t st_main = st;
     st = st_ring;
-    if (ctx->rd_variant == 4 && dp.curbPoints == 5)        // four positions per thread (default curb_points only)
-      K("k_ring_detect4", k_ring_detect4<4><<<gtile, 256, 0, st>>>(buf, dp, S));
-    else if (ctx->rd_variant == 45 && dp.curbPoints == 5) K("k_ring_detect4", k_ring_detect4<5><<<gtile, 256, 0, st>>>(buf, dp, S));
-    else if (ctx->rd_variant == 46 && dp.curbPoints == 5) K("k_ring_detect4", k_ring_detect4<6><<<gtile, 256, 0, st>>>(buf, dp, S));
-    else if (ctx->rd_variant == 6) K("k_ring_detect", k_ring_detect<6><<<gpts, 256, 0, st>>>(buf, dp, S));
-    else if (ctx->rd_variant == 5) K("k_ring_detect", k_ring_detect<5><<<gpts, 256, 0, st>>>(buf, dp, S));
-    else K("k_ring_detect", k_ring_detect<8><<<gpts, 256, 0, st>>>(buf, dp, S));   // 8 CTAs/SM (32 registers)
+    if (dp.curbPoints == 5) K("k_ring_detect4", k_ring_detect4<<<gtile, 256, 0, st>>>(buf, dp, S));   // four positions per thread
+    else K("k_ring_detect", k_ring_detect<<<gpts, 256, 0, st>>>(buf, dp, S));                        // one position per thread
     st = st_main;
   }
   if (fork) CK(cudaEventRecord(ctx->ev_sjoin[side], st_ring));
   if (dp.star) {
     const int gbig = std::max(4, std::min(kSectKeys, 2048 / B));
     const dim3 gscan((kSectKeys + kScanWarps * 32 - 1) / (kScanWarps * 32), B);
-    if (ctx->sort_variant == 16) K("k_star_sort_warp", k_star_sort_warp<16><<<dim3(kSectKeys, B), 32, 0, st>>>(buf, dp, S));
-    else K("k_star_sort_warp", k_star_sort_warp<32><<<dim3(kSectKeys, B), 32, 0, st>>>(buf, dp, S));
+    K("k_star_sort_warp", k_star_sort_warp<<<dim3(kSectKeys, B), 32, 0, st>>>(buf, dp, S));
     K("k_star_sort_big", k_star_sort_big<<<dim3(gbig, B), 256, kStarCtaSmem, st>>>(buf, dp, S));
     K("k_star_scan", k_star_scan<<<gscan, kScanWarps * 32, 0, st>>>(buf, dp, S));
     if (dp.star_prefix)            // sectors whose edge search ran off the near-first prefix: full sort, search resumed
@@ -208,13 +187,13 @@ int launch_pipeline(urf_ctx* ctx, const DevBuffers& buf, int B, int S, bool want
   K("k_reach", k_reach<<<dim3((2 * kDegBins + 7) / 8, B), 256, 0, st>>>(buf, dp));
   K("k_tab2", k_tab2<<<dim3((dp.channels + kTab2Rings - 1) / kTab2Rings, B), kTab2Rings * 64, 0, st>>>(buf, dp));
   K("k_label", k_label<<<gpts, 256, 0, st>>>(buf, dp, S));
-  if (ctx->markers_variant == 2 || (ctx->markers_variant == 1 && S > kMarkSingleMax)) {   // large scans: a grid of CTAs per scan, three launches
+  if (S <= kMarkSingleMax) K("k_markers1", k_markers1<<<dim3(1, B), kMark1Threads, 0, st>>>(buf, S));   // one CTA per scan
+  else {                                                      // large scans: a grid of CTAs per scan, three launches
     const dim3 gm(std::max(1, std::min(64, S / 16384)), B);
     K("k_markers_grid1", k_markers_grid<1><<<gm, kMarkGridThreads, 0, st>>>(buf, S));
     K("k_markers_grid2", k_markers_grid<2><<<gm, kMarkGridThreads, 0, st>>>(buf, S));
     K("k_verts", k_verts<<<B, 384, 0, st>>>(buf, S));
-  } else if (ctx->markers_variant == 1) K("k_markers1", k_markers1<<<dim3(1, B), kMark1Threads, 0, st>>>(buf, S));   // one CTA per scan
-  else K("k_markers", k_markers<<<dim3(kMarkCtas, B), kMarkThreads, 0, st>>>(buf, S));              // cluster of kMarkCtas CTAs per scan
+  }
   if (want_order) K("k_sort_rings", k_sort_rings<<<dim3(dp.channels, B), kSortThreads, kRingSmemKeys * sizeof(unsigned long long), st>>>(buf, S));
 #undef K
   if (last) CK(cudaEventRecord(ctx->ev1, st));
@@ -395,11 +374,8 @@ int urf_create(urf_ctx** out, int device, int max_points, int max_batch) {
   CKF(cudaFuncSetAttribute(k_star_refine, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStarCtaSmem));
   CKF(cudaFuncSetAttribute(k_sort_rings, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kRingSmemKeys * sizeof(unsigned long long))));
   urf_default_params(&ctx->params);
-  const char* fe = std::getenv("URF_FORCE_EXACT_REGISTRATION");
-  narrow_params(&ctx->params, &ctx->dp, ctx->dp.Kfi, fe && fe[0] == '1', 0);
-  const char* sp = std::getenv("URF_STAR_PREFIX");          // near-first star sort, on unless URF_STAR_PREFIX=0 (A/B measurements)
-  ctx->dp.star_prefix = !(sp && sp[0] == '0');
-  ctx->dp.star_pivot = 17;
+  narrow_params(&ctx->params, &ctx->dp, ctx->dp.Kfi, 0, 0);
+  ctx->dp.star_prefix = 1;                                  // near-first star sort
 #undef TRY
 #undef CKF
   *out = ctx;
@@ -417,7 +393,6 @@ void urf_destroy(urf_ctx* ctx) {
   if (ctx->h_out) cudaFreeHost(ctx->h_out);
   if (ctx->h_packtot) cudaFreeHost(ctx->h_packtot);
   if (ctx->gexec) cudaGraphExecDestroy(ctx->gexec);
-  if (ctx->bexec) cudaGraphExecDestroy(ctx->bexec);
   for (cudaEvent_t e : ctx->kev) cudaEventDestroy(e);
   for (cudaEvent_t e : ctx->ev_in) cudaEventDestroy(e);
   for (cudaEvent_t e : ctx->ev_comp) cudaEventDestroy(e);
@@ -460,28 +435,25 @@ int urf_get_params(const urf_ctx* ctx, urf_params* p) {
 }
 
 // test/diagnostic options: 0 = force exact ring registration (0/1); 1 = per-kernel CUDA-event timing (slots, 0 = off);
-// 2 = number of compute streams a device-resident batch is spread over (1..4); 3 = CUDA graph for small batches (0/1);
-// 4 = near-first star sort (0/1, default 1); 5 = scans per sub-batch of a device-resident batch (0 = batch / streams);
-// 6 = replay the fork/join of a device-resident batch as one CUDA graph (0/1); 7 = sub-batches of a stream share one
-// workspace slot (0/1); 8 = ring detector variant; 9 = marker search variant; 10 = near-first pivot rank (3..28 of 32 samples);
-// 11 = ring detector on a side stream next to the star-shaped search (0/1, default 1); 12 = widest single-warp star sort
-// network in elements per lane (16 default, or 32)
+// 2 = number of compute streams a device-resident batch is spread over (1..16); 3 = CUDA graph for small batches (0/1);
+// 4 = near-first star sort (0/1, default 1).
+// Options 5-12 selected tuning variants that were measured slower and removed (DESIGN.md §6). Each still accepts the
+// value that is now built in, so existing settings keep working, and rejects any other value:
+// 5 scans per sub-batch (0 = batch / streams), 6 batch CUDA graph (0), 7 shared workspace slot (0), 8 ring detector
+// (46: k_ring_detect4 at 6 CTAs/SM for curb_points 5, else k_ring_detect), 9 marker search (1: one CTA per scan up to
+// kMarkSingleMax points, else a grid), 10 near-first pivot rank (kStarPivot), 11 ring detector on a side stream (1),
+// 12 widest single-warp star sort network (16 elements per lane).
 int urf_set_option(urf_ctx* ctx, int option, int value) {
   if (!ctx) return URF_ERR_INVALID;
+  static constexpr int kRetired[][2] = {{5, 0}, {6, 0}, {7, 0}, {8, 46}, {9, 1}, {10, kStarPivot}, {11, 1}, {12, 16}};
+  for (const auto& r : kRetired)
+    if (option == r[0]) return value == r[1] ? URF_OK : URF_ERR_INVALID;
   CK(cudaSetDevice(ctx->device));
   ctx->version++;
   if (option == 0) { ctx->dp.force_exact = value != 0; ctx->version++; return URF_OK; }
   if (option == 4) { ctx->dp.star_prefix = value != 0; ctx->version++; return URF_OK; }
   if (option == 3) { ctx->use_graph = value != 0; return URF_OK; }
   if (option == 2) { ctx->groups = value < 1 ? 1 : (value > urf_ctx::kGroups ? urf_ctx::kGroups : value); return URF_OK; }
-  if (option == 5) { ctx->sub = value < 0 ? 0 : value; return URF_OK; }
-  if (option == 6) { ctx->batch_graph = value != 0; return URF_OK; }
-  if (option == 7) { ctx->slot_reuse = value != 0; return URF_OK; }
-  if (option == 8) { ctx->rd_variant = value; return URF_OK; }
-  if (option == 9) { ctx->markers_variant = value; return URF_OK; }
-  if (option == 12) { ctx->sort_variant = value == 16 ? 16 : 32; return URF_OK; }
-  if (option == 11) { ctx->inner_fork = value != 0; return URF_OK; }
-  if (option == 10) { ctx->dp.star_pivot = value < 3 ? 3 : (value > 28 ? 28 : value); return URF_OK; }
   if (option == 1) {                   // value = number of event slots (0 = off)
     CK(cudaStreamSynchronize(ctx->stream));               // events of the previous setting may still be pending
     if (ctx->gexec) { cudaGraphExecDestroy(ctx->gexec); ctx->gexec = nullptr; ctx->g_B = -1; }
@@ -556,56 +528,27 @@ int urf_enqueue_batch_device_ex(urf_ctx* ctx, const float* d_xyzi, int stride_po
   if (want_order) bufv.order = d_order;
   int rc = URF_OK;
   const int T = (stride_points + kChunk - 1) / kChunk;
-  int sub = ctx->sub > 0 ? std::min(ctx->sub, batch) : (batch + ctx->groups - 1) / ctx->groups;
-  const int nsub = (batch + sub - 1) / sub;
-  const int G = (ctx->profile || batch < 2 * ctx->groups) ? 1 : std::min(ctx->groups, nsub);   // per-kernel event timing needs one stream
+  const int sub = (batch + ctx->groups - 1) / ctx->groups;    // scans per stream
+  const int G = (ctx->profile || batch < 2 * ctx->groups) ? 1 : (batch + sub - 1) / sub;   // per-kernel event timing needs one stream
   if (G == 1) rc = launch_pipeline(ctx, bufv, batch, stride_points, want_order);
   else {
-    // fork: the ctx stream hands sub-batches to the group streams (round-robin) and joins them again, so callers still see
-    // ONE stream. Scans are independent: a stream works through its sub-batches one after the other.
-    const bool reuse = ctx->slot_reuse;
-    auto fork_join = [&]() -> int {
-      CK(cudaEventRecord(ctx->ev_fork, ctx->stream));
-      int launches = 0;
-      for (int g = 0; g < G; g++) CK(cudaStreamWaitEvent(ctx->s_grp[g], ctx->ev_fork, 0));
-      for (int j = 0; j < nsub; j++) {
-        const int g = j % G, b0 = j * sub, nb = std::min(sub, batch - b0);
-        const int r = launch_pipeline(ctx, slot_view(bufv, b0, reuse ? g * sub : b0, stride_points, T, ctx->dp.channels), nb, stride_points,
-                                      want_order, false, false, ctx->s_grp[g]);
-        if (r != URF_OK) return r;
-        launches += ctx->launches;
-      }
-      for (int g = 0; g < G; g++) {
-        CK(cudaEventRecord(ctx->ev_join[g], ctx->s_grp[g]));
-        CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_join[g], 0));
-      }
-      ctx->launches = launches;
-      return URF_OK;
-    };
+    // fork: the ctx stream hands one sub-batch to each group stream and joins them again, so callers still see ONE stream
     CK(cudaEventRecord(ctx->ev0, ctx->stream));
-    if (!ctx->batch_graph) rc = fork_join();
-    else {
-      auto& k = ctx->bkey;
-      if (!ctx->bexec || k.B != batch || k.S != stride_points || k.sub != sub || k.G != G || k.order != (int)want_order || k.reuse != reuse ||
-          k.in != (const void*)d_xyzi || k.label != (void*)d_label || k.orderp != (void*)d_order || k.version != ctx->version) {
-        if (ctx->bexec) { cudaGraphExecDestroy(ctx->bexec); ctx->bexec = nullptr; }
-        cudaGraph_t graph = nullptr;
-        CK(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
-        rc = fork_join();
-        const cudaError_t e = cudaStreamEndCapture(ctx->stream, &graph);
-        if (rc != URF_OK || e != cudaSuccess || !graph) {
-          if (graph) cudaGraphDestroy(graph);
-          if (rc == URF_OK) { ctx->err = std::string("batch graph capture: ") + cudaGetErrorString(e); rc = URF_ERR_CUDA; }
-        } else {
-          const cudaError_t ei = cudaGraphInstantiate(&ctx->bexec, graph, 0);
-          cudaGraphDestroy(graph);
-          if (ei != cudaSuccess) { ctx->bexec = nullptr; ctx->err = cudaGetErrorString(ei); rc = URF_ERR_CUDA; }
-          else { k.B = batch; k.S = stride_points; k.sub = sub; k.G = G; k.order = (int)want_order; k.reuse = reuse; k.in = d_xyzi; k.label = d_label; k.orderp = d_order;
-                 k.version = ctx->version; k.launches = ctx->launches; }
-        }
-      }
-      if (rc == URF_OK) { CK(cudaGraphLaunch(ctx->bexec, ctx->stream)); ctx->launches = ctx->bkey.launches; }
+    CK(cudaEventRecord(ctx->ev_fork, ctx->stream));
+    int launches = 0;
+    for (int g = 0; g < G; g++) {
+      const int b0 = g * sub;
+      CK(cudaStreamWaitEvent(ctx->s_grp[g], ctx->ev_fork, 0));
+      rc = launch_pipeline(ctx, offset_view(bufv, b0, stride_points, T, ctx->dp.channels), std::min(sub, batch - b0), stride_points,
+                           want_order, false, false, ctx->s_grp[g]);
+      if (rc != URF_OK) break;
+      launches += ctx->launches;
     }
+    for (int g = 0; g < G; g++) {
+      CK(cudaEventRecord(ctx->ev_join[g], ctx->s_grp[g]));
+      CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_join[g], 0));
+    }
+    ctx->launches = launches;
     CK(cudaEventRecord(ctx->ev1, ctx->stream));
   }
   ctx->last_B = batch; ctx->last_S = stride_points;

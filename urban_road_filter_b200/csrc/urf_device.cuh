@@ -47,8 +47,12 @@ struct DevParams {
   int force_exact;   // test hook: always use the exact registration path
   int want_order;    // produce emission order (per-ring azimuth sort)
   int star_prefix;   // near-first star sort on (default); 0 = always sort whole sectors (test hook)
-  int star_pivot;    // near-first pivot: rank (0..31) of the pivot among 32 evenly spaced radius samples (default 17: the 18th smallest)
 };
+
+// Near-first star sort: rank (0..31) of the pivot among 32 evenly spaced radius samples of a sector, here the 18th
+// smallest (tighter and looser pivots measured slower or equal, DESIGN.md §6). The eight-warp sort takes rank
+// 8 * kStarPivot + 7 of 256 samples.
+constexpr int kStarPivot = 17;
 
 // Small per-scan outputs copied back to the host after every call.
 struct ScanOut {

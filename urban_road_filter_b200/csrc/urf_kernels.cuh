@@ -9,11 +9,11 @@
 //   k_reset -> k_points -> k_register -> k_assign -> k_scan_offsets (+ exact re-registration of refuted scans)
 //   -> k_scatter -> k_star_sort_warp (near-first) -> k_star_sort_big (large sectors, exact fallback) -> k_star_scan
 //   -> k_star_refine (sectors without an edge in their prefix: full sort, walk resumed)
-//   -> k_ring_detect -> k_tab1 -> k_reach -> k_tab2 -> k_label (input order) -> k_markers (cluster of 8 CTAs per scan)
+//   -> k_ring_detect4 / k_ring_detect (on a side stream, next to the star-shaped search) -> k_tab1 -> k_reach -> k_tab2
+//   -> k_label (input order) -> k_markers1 (one CTA per scan; scans above 300 k points: k_markers_grid x 2 -> k_verts)
 //   [-> k_sort_rings when the emission order is requested]
 //   PointCloud2 entry points: k_unpack_cloud2 in front, k_pack_count -> k_pack_scan -> k_pack_write behind
 #pragma once
-#include <cooperative_groups.h>
 #include <type_traits>
 
 #include "urf_device.cuh"
@@ -21,8 +21,6 @@
 #include "urf_stdsort.cuh"
 
 namespace urf {
-
-namespace cg = cooperative_groups;
 
 __constant__ float c_beam_d[kSectKeys];
 __constant__ float c_beam_o[kSectKeys];
@@ -754,14 +752,14 @@ __device__ __forceinline__ int select_far(const float4* __restrict__ src, int n,
 // without an edge is put on tab.refine and redone in full (k_star_refine: full sort + star_resume_walk). Exact either
 // way: every point of the prefix is closer than every point behind it.
 constexpr int kPrefixMin = 128;
-// MAXEPL = 32: every sector of up to kWarpCap points is sorted here (128 registers, 16 warps per SM). MAXEPL = 16: sorts
-// of more than 512 elements go to k_star_sort_big's list instead, which leaves this kernel with the networks of up to 16
-// elements per lane (fewer registers, more resident warps to hide the shuffle latency). (Measured and dropped: a keys-only
-// network — one SHFL + two VIMNMX per remote compare-exchange instead of two SHFL, a compare and two selects — with the
-// payload recovered by a binary search of every key in the sorted keys: 30 % fewer instructions, but 0.7 % slower per step.)
-template <int MAXEPL>
-__global__ void __launch_bounds__(32, MAXEPL >= 32 ? 16 : 32) k_star_sort_warp(DevBuffers buf, DevParams prm, int S) {
-  constexpr int kList = 32 * MAXEPL;                                    // longest list this kernel sorts itself
+// Sorts of more than 512 elements go to k_star_sort_big's list, which leaves this kernel with the networks of up to 16
+// elements per lane (64 registers, 32 resident warps per SM to hide the shuffle latency; measured and dropped: networks
+// of up to 32 elements per lane here, 128 registers and 16 warps per SM, 2 % slower per step at C2 x 128). (Also measured
+// and dropped: a keys-only network — one SHFL + two VIMNMX per remote compare-exchange instead of two SHFL, a compare and
+// two selects — with the payload recovered by a binary search of every key in the sorted keys: 30 % fewer instructions,
+// but 0.7 % slower per step.)
+__global__ void __launch_bounds__(32, 32) k_star_sort_warp(DevBuffers buf, DevParams prm, int S) {
+  constexpr int kList = 32 * 16;                                        // longest list this kernel sorts itself
   __shared__ unsigned s_pk[kList], s_pe[kList];
   const int b = blockIdx.y, s = blockIdx.x, lane = threadIdx.x;
   ScanTab& tab = buf.tab[b];
@@ -781,25 +779,23 @@ __global__ void __launch_bounds__(32, MAXEPL >= 32 ? 16 : 32) k_star_sort_warp(D
   bool tie;
   int m = 0;
   if (prm.star_prefix && n > kPrefixMin) {
-    if (n <= 256) m = select_near<8>(src, n, lane, s_pk, s_pe, prm.star_pivot, kList);
-    else if (n <= 512) m = select_near<16>(src, n, lane, s_pk, s_pe, prm.star_pivot, kList);
-    else m = select_near<32>(src, n, lane, s_pk, s_pe, prm.star_pivot, kList);
+    if (n <= 256) m = select_near<8>(src, n, lane, s_pk, s_pe, kStarPivot, kList);
+    else if (n <= 512) m = select_near<16>(src, n, lane, s_pk, s_pe, kStarPivot, kList);
+    else m = select_near<32>(src, n, lane, s_pk, s_pe, kStarPivot, kList);
   }
   const bool near = m >= 32 && 4 * m <= 3 * n;                          // worth it: sort the near part only
-  if (MAXEPL < 32 && (near ? m : n) > 32 * MAXEPL) {                    // a wide network: eight warps do it (k_star_sort_big)
+  if ((near ? m : n) > kList) {                                         // a wide network: eight warps do it (k_star_sort_big)
     if (lane == 0) tab.biglist[atomicAdd(&tab.nbig, 1)] = (unsigned short)s;
     return;
   }
   if (near) {
     if (m <= 128) tie = bitonic_sector<4, 1, true>(src, dst, m, lane, s_pk, s_pe);
     else if (m <= 256) tie = bitonic_sector<8, 1, true>(src, dst, m, lane, s_pk, s_pe);
-    else if (MAXEPL >= 32 && m > 512) tie = bitonic_sector<32, 1, true>(src, dst, m, lane, s_pk, s_pe);
     else tie = bitonic_sector<16, 1, true>(src, dst, m, lane, s_pk, s_pe);
     if (lane == 0) tab.sorted_len[s] = m;
   } else {
     if (n <= 128) tie = bitonic_sector<4, 1>(src, dst, n, lane, nullptr, nullptr);
     else if (n <= 256) tie = bitonic_sector<8, 1>(src, dst, n, lane, nullptr, nullptr);
-    else if (MAXEPL >= 32 && n > 512) tie = bitonic_sector<32, 1>(src, dst, n, lane, nullptr, nullptr);
     else tie = bitonic_sector<16, 1>(src, dst, n, lane, nullptr, nullptr);
   }
   if (__any_sync(0xffffffffu, tie) && lane == 0) tab.slowlist[atomicAdd(&tab.nslow, 1)] = (unsigned short)s;   // sets F_TIE_SECTOR there
@@ -907,9 +903,9 @@ __global__ void __launch_bounds__(256) k_star_sort_big(DevBuffers buf, DevParams
     if (threadIdx.x == 0) s_tie = 0;
     int m = 0;
     if (prm.star_prefix) {
-      if (n <= 2048) m = select_near_cta<8>(src, n, threadIdx.x, s_xk, s_xe, s_misc, 8 * prm.star_pivot + 7);
-      else if (n <= 4096) m = select_near_cta<16>(src, n, threadIdx.x, s_xk, s_xe, s_misc, 8 * prm.star_pivot + 7);
-      else m = select_near_cta<32>(src, n, threadIdx.x, s_xk, s_xe, s_misc, 8 * prm.star_pivot + 7);
+      if (n <= 2048) m = select_near_cta<8>(src, n, threadIdx.x, s_xk, s_xe, s_misc, 8 * kStarPivot + 7);
+      else if (n <= 4096) m = select_near_cta<16>(src, n, threadIdx.x, s_xk, s_xe, s_misc, 8 * kStarPivot + 7);
+      else m = select_near_cta<32>(src, n, threadIdx.x, s_xk, s_xe, s_misc, 8 * kStarPivot + 7);
     }
     const bool near = m >= 256 && 4 * m <= 3 * n;                          // uniform: m comes from shared memory
     const bool tie = near ? sort_sector_cta<true>(src, dst, m, threadIdx.x, s_xk, s_xe) : sort_sector_cta<false>(src, dst, n, threadIdx.x, s_xk, s_xe);
@@ -1165,9 +1161,9 @@ __global__ void __launch_bounds__(kScanWarps * 32) k_star_scan(DevBuffers buf, D
 // so every thread evaluates only the gates and the CTA compacts the survivors into a work list that full warps then run
 // the angle tests over (x-zero items from thread 0 upwards, z-zero items from thread 255 downwards). Points found to be
 // curb points are marked in input order and entered into the curb bins (curb_hit); nothing else is written per point.
+// Runs for curb_points other than the default 5 (k_ring_detect4 below takes that), eight CTAs per SM (32 registers).
 constexpr int kHalo = 32;
-template <int MINB>
-__global__ void __launch_bounds__(256, MINB) k_ring_detect(DevBuffers buf, DevParams prm, int S) {
+__global__ void __launch_bounds__(256, 8) k_ring_detect(DevBuffers buf, DevParams prm, int S) {
   const int b = blockIdx.y;
   const ScanOut& out = buf.out[b];
   const int p0 = blockIdx.x * 256, tid = threadIdx.x, p = p0 + tid;
@@ -1213,7 +1209,7 @@ __global__ void __launch_bounds__(256, MINB) k_ring_detect(DevBuffers buf, DevPa
       const int off = base - (p0 - kHalo);                // ring-local index q lives at tile slot off + q
       const RingSoA ring{s_x + off, s_y + off, s_z + off};
       need_x = prm.x_zero && xzero_pre(prm, ring, n, m);
-      need_z = prm.z_zero && (prm.curbPoints == 5 ? zzero_pre_t<5>(prm, ring, n, m) : zzero_pre_t<0>(prm, ring, n, m));
+      need_z = prm.z_zero && zzero_pre_t<0>(prm, ring, n, m);
     } else {                                              // huge curb_points: straight from global memory
       const float4* ring = bucket + base;
       hit = (prm.x_zero && xzero_mark(prm, ring, n, m, buf.newY)) ||                  // x_zero_method.cpp:66
@@ -1241,7 +1237,7 @@ __global__ void __launch_bounds__(256, MINB) k_ring_detect(DevBuffers buf, DevPa
     for (int it = 255 - tid; it < nz; it += 256) {                      // z-zero angle tests, z_zero_method.cpp:23-66
       const int t = s_item[511 - it], base = s_base[t], off = base - (p0 - kHalo);
       const RingSoA ring{s_x + off, s_y + off, s_z + off};
-      if (prm.curbPoints == 5 ? zzero_post_t<5>(prm, ring, p0 + t - base) : zzero_post_t<0>(prm, ring, p0 + t - base)) s_hit[t] = 1;
+      if (zzero_post_t<0>(prm, ring, p0 + t - base)) s_hit[t] = 1;
     }
     __syncthreads();
     hit = act && s_hit[tid];                                            // x_zero_method.cpp:66, z_zero_method.cpp:71
@@ -1264,9 +1260,9 @@ __global__ void __launch_bounds__(256, MINB) k_ring_detect(DevBuffers buf, DevPa
 // side (z-zero) and at -2 / +3 (x-zero). Four consecutive positions share a window of 14 heights, which the thread fetches
 // with five 16-byte shared-memory loads instead of 4 x 14 scalar ones; ring lookup, work-list compaction and the maximum of
 // the planar sums are amortised over the four positions as well. Same logic functions, same results as k_ring_detect.
+// Six CTAs per SM (40 registers; measured 1.337 ms per step against 1.351 at five and 1.380 at four).
 constexpr int kTile4 = 1024;
-template <int MINB>
-__global__ void __launch_bounds__(256, MINB) k_ring_detect4(DevBuffers buf, DevParams prm, int S) {
+__global__ void __launch_bounds__(256, 6) k_ring_detect4(DevBuffers buf, DevParams prm, int S) {
   constexpr int CP = 5;
   const int b = blockIdx.y;
   const ScanOut& out = buf.out[b];
@@ -1597,106 +1593,15 @@ __global__ void __launch_bounds__(256) k_label(DevBuffers buf, DevParams prm, in
         make_uint4((unsigned)bin | ((unsigned)k << 16), fbits(a), fbits(d), (unsigned)i);
 }
 
-// k_markers: marker candidate vertices, lidar_segmentation.cpp:305-351, over the road points k_label listed (32 slots per
-// warp of input points, count in roadcnt) — one thread-block CLUSTER of kMarkCtas CTAs per scan. Every CTA aggregates its
-// share of the list per degree bin in its own shared memory, then merges into the arrays of the cluster's first CTA
-// through distributed shared memory (cluster.map_shared_rank); the passes are separated by cluster barriers:
+// k_markers1: marker candidate vertices, lidar_segmentation.cpp:305-351, over the road points k_label listed (32 slots per
+// warp of input points, count in roadcnt) — ONE CTA of 1024 threads per scan, everything in its own shared memory:
 //   pass 1  farthest candidate road point per bin (candidates: road points scanned before the bin's first non-road point)
 //   pass 2  first candidate in scan order that reaches that distance (`d > maxDistanceRoad` is strict, :329)
-//   then    the first CTA compacts the per-bin winners in bin order into markerPointsArray (:343-350)
-constexpr int kMarkCtas = 8, kMarkThreads = 256;
-__global__ void __cluster_dims__(kMarkCtas, 1, 1) __launch_bounds__(kMarkThreads) k_markers(DevBuffers buf, int S) {
-  cg::cluster_group cluster = cg::this_cluster();
-  const int b = blockIdx.y;
-  ScanOut& out = buf.out[b];
-  const ScanTab& tab = buf.tab[b];
-  __shared__ unsigned long long s_cut[kDegBins];       // first-non-road keys of the scan (read only here)
-  __shared__ unsigned s_dmax[kDegBins];                // this CTA's share; in CTA 0 also the merged result
-  __shared__ unsigned s_far[kDegBins];                 // copy of the merged result for pass 2
-  __shared__ unsigned long long s_best[kDegBins];      // this CTA's share; in CTA 0 also the merged result
-  __shared__ int s_wsum[kMarkThreads / 32];
-  unsigned* dmax0 = cluster.map_shared_rank(s_dmax, 0);
-  unsigned long long* best0 = cluster.map_shared_rank(s_best, 0);
-  const int tid = threadIdx.x;
-  for (int t = tid; t < kDegBins; t += kMarkThreads) { s_cut[t] = tab.cutbest[t]; s_dmax[t] = 0u; s_best[t] = ~0ull; }
-  cluster.sync();                                      // every CTA's arrays are initialised before anybody merges into CTA 0's
-  const int n = buf.n[b];
-  const int nseg = (n + 31) >> 5;                      // one list segment per warp of input points
-  const unsigned gb = scan_base(b, S);
-  const unsigned char* cnt = buf.roadcnt + (size_t)b * ((S + 31) >> 5);
-  const uint4* list = buf.roadlist + gb;
-  constexpr int STEP = kMarkCtas * kMarkThreads;
-  const int t0 = blockIdx.x * kMarkThreads + tid;
-  for (int seg = t0; seg < nseg; seg += STEP) {        // a thread walks the segments it owns, four entries in flight
-    const int c = cnt[seg];
-    for (int r0 = 0; r0 < c; r0 += 4) {
-      uint4 e[4];
-#pragma unroll
-      for (int u = 0; u < 4; u++) e[u] = list[seg * 32 + min(r0 + u, c - 1)];
-#pragma unroll
-      for (int u = 0; u < 4; u++) {
-        if (r0 + u >= c) break;
-        const int bin = e[u].x & 0xffff, k = e[u].x >> 16;
-        if (marker_candidate(s_cut[bin], k, e[u].y, (int)e[u].w) && s_dmax[bin] < e[u].z) atomicMax(&s_dmax[bin], e[u].z);
-      }
-    }
-  }
-  __syncthreads();
-  if (blockIdx.x != 0)
-    for (int t = tid; t < kDegBins; t += kMarkThreads) { const unsigned v = s_dmax[t]; if (v) atomicMax(&dmax0[t], v); }
-  cluster.sync();
-  for (int t = tid; t < kDegBins; t += kMarkThreads) s_far[t] = dmax0[t];
-  __syncthreads();
-  for (int seg = t0; seg < nseg; seg += STEP) {
-    const int c = cnt[seg];
-    for (int r0 = 0; r0 < c; r0 += 4) {
-      uint4 e[4];
-#pragma unroll
-      for (int u = 0; u < 4; u++) e[u] = list[seg * 32 + min(r0 + u, c - 1)];
-#pragma unroll
-      for (int u = 0; u < 4; u++) {
-        if (r0 + u >= c) break;
-        const int bin = e[u].x & 0xffff, k = e[u].x >> 16;
-        if (e[u].z != 0u && e[u].z == s_far[bin] && marker_candidate(s_cut[bin], k, e[u].y, (int)e[u].w)) {
-          const unsigned long long key = best_key(k, e[u].y, (int)e[u].w);
-          if (s_best[bin] > key) atomicMin(&s_best[bin], key);
-        }
-      }
-    }
-  }
-  __syncthreads();
-  if (blockIdx.x != 0)
-    for (int t = tid; t < kDegBins; t += kMarkThreads) { const unsigned long long v = s_best[t]; if (v != ~0ull) atomicMin(&best0[t], v); }
-  cluster.sync();                                      // the other CTAs are done with CTA 0's shared memory
-  if (blockIdx.x != 0) return;
-  int run = 0;                                         // vertices written so far (bins are compacted in bin order)
-  for (int c0 = 0; c0 < kDegBins; c0 += kMarkThreads) {
-    const int i = c0 + tid;
-    const bool has = i < kDegBins && s_best[i] != ~0ull;
-    const unsigned bal = __ballot_sync(0xffffffffu, has);
-    const int warp = tid >> 5, lane = lane_id();
-    if (lane == 0) s_wsum[warp] = __popc(bal);
-    __syncthreads();
-    int off = 0, total = 0;
-    for (int w = 0; w < kMarkThreads / 32; w++) { if (w < warp) off += s_wsum[w]; total += s_wsum[w]; }
-    if (has) {
-      const int slot = run + off + __popc(bal & ((1u << lane) - 1u));
-      const int p = (int)(s_best[i] & 0xffffffull);    // input index of the winner
-      const float4 q = buf.in[(size_t)b * S + p];
-      out.vert[slot][0] = q.x; out.vert[slot][1] = q.y; out.vert[slot][2] = q.z;
-      out.vert[slot][3] = s_cut[i] != ~0ull ? 1.0f : 0.0f;              // redPoints, :320,348
-    }
-    run += total;
-    __syncthreads();
-  }
-  if (tid == 0) out.n_vert = run;
-  for (int i = run + tid; i < URF_MAX_VERTS; i += kMarkThreads) { out.vert[i][0] = 0.f; out.vert[i][1] = 0.f; out.vert[i][2] = 0.f; out.vert[i][3] = 0.f; }   // defined tail
-}
-
-// k_markers1: the same search by ONE CTA of 1024 threads per scan, everything in its own shared memory (no cluster, no
-// distributed shared memory): a warp takes 32 list segments at a time, scans their counts and spreads the entries evenly
-// over its lanes (entry e of the 32 segments belongs to the segment whose exclusive count prefix is the last one <= e), four
-// entries in flight per lane. Selected with option 9; bench.py's tuning sweep compares the two.
+//   then    the per-bin winners are compacted in bin order into markerPointsArray (:343-350)
+// In a pass a warp takes 32 list segments at a time, scans their counts and spreads the entries evenly over its lanes
+// (entry e of the 32 segments belongs to the segment whose exclusive count prefix is the last one <= e), four entries in
+// flight per lane. (Measured and dropped: a cluster of eight CTAs per scan merging through distributed shared memory,
+// 0.077 ms against 0.052 ms, its cluster barriers dominating the stall samples.)
 constexpr int kMark1Threads = 1024;
 template <int PASS>
 __device__ __forceinline__ void markers_pass(const uint4* __restrict__ list, const unsigned char* __restrict__ cnt, int nseg,
